@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark (BASELINE.json): 3-D Navier-Stokes FNO training step, samples/s.
 
-    python bench.py --gpus N --steps K --warmup W [--impl fused|baseline|reference]
+    python bench.py --gpus N --steps K --warmup W [--impl fused|baseline|reference] [--dump-outputs DIR]
 
 Config: global field 128^3 x 20 t, width 20, modes (12,12,12,10), 4 Fourier blocks, batch 1,
 input [1,1,128,128,128,1] -> output [1,1,128,128,128,20]; 1 x N y-pencil over N GPUs (strong
@@ -58,7 +58,39 @@ def parse():
     ap.add_argument("--no-graph", action="store_true", help="launch every kernel eagerly instead of replaying a CUDA graph")
     ap.add_argument("--no-parity", action="store_true",
                     help="skip the N-rank vs 1-rank output / loss comparison that rank 0 runs after the timed regions")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one produced as DIR/<name>.npy: its loss and the "
+                         "updated parameters in the canonical (partition-independent) layout; see dump_outputs()")
     return ap.parse_args()
+
+
+DUMP_LIMIT = 64 * 10 ** 6    # bytes, all files of --dump-outputs together
+
+
+def dump_outputs(out_dir, arrays):
+    """Write ``{name: tensor}`` as ``out_dir/<name>.npy`` so that two builds can be compared output for output.
+
+    float64 stays float64, every other dtype becomes float32; a complex tensor gains a trailing axis of 2 (real,
+    imaginary).  All files together stay within ``DUMP_LIMIT``: arrays are written smallest first, each may take an
+    equal share of what is left, and one larger than its share is replaced by a sample of that many elements of its
+    flattened form, at sorted indices drawn from a generator seeded with 0 -- the same elements for the same
+    arguments, run after run."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    out = {}
+    for name, t in arrays.items():
+        t = t.detach().cpu()
+        if t.is_complex():
+            t = torch.view_as_real(t)
+        out[name] = (t.double() if t.dtype == torch.float64 else t.float()).numpy()
+    left = DUMP_LIMIT - 4096 * len(out)                  # room for the .npy headers
+    for i, (name, a) in enumerate(sorted(out.items(), key=lambda kv: kv[1].nbytes)):
+        n = left // (len(out) - i) // a.itemsize
+        if a.size > n:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, n, replace=False, shuffle=False))]
+        left -= a.nbytes
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 class ClockSampler:
@@ -132,6 +164,7 @@ def main():
     import torch.distributed as dist
     import dfno_b200 as d
     from dfno_b200.parallel.decomposition import assemble_slices, shard_bounds
+    from dfno_b200.utils.checkpoint import gather_global_state
     from dfno_b200.utils.env import ensure_process_group
 
     N = args.gpus
@@ -259,6 +292,10 @@ def main():
     ms_step = total_ms / args.steps
     value = args.batch * 1000.0 / ms_step
     loss_value = float(last_loss)
+    if args.dump_outputs:
+        state = gather_global_state(net)                     # collective; the canonical state lands on rank 0
+        if rank == 0:
+            dump_outputs(args.dump_outputs, {"loss": last_loss, **state})
 
     # ---- end to end through the public Trainer API: pinned host batch in, loss out
     e2e = None

@@ -8,6 +8,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 from dfno_b200.utils.testing import free_port
@@ -95,3 +96,45 @@ def test_bench_contract_dry_run():
             assert key in rec, key
         assert rec["n_gpus"] == 2 and rec["steps"] == 2 and rec["warmup"] == 3 and rec["impl"] == impl
         assert "h2d_bytes_per_step" in rec["e2e"] and rec["value"] > 0      # bytes are 0 in the CPU dry run
+
+
+def test_bench_dump_outputs_dry_run(tmp_path):
+    """--dump-outputs: the loss of the last timed step and the updated canonical parameters, the same from run to
+    run with the same arguments."""
+    small = ["--device", "cpu", "--grid", "16", "--nt", "8", "--width", "4", "--modes", "2", "2", "2", "2",
+             "--blocks", "1", "--steps", "2", "--warmup", "3", "--no-e2e"]
+    dumps = []
+    for i in range(2):
+        out = _run(["bench.py", "--gpus", "2", "--impl", "baseline", *small, "--dump-outputs", str(tmp_path / str(i))])
+        rec = json.loads([l for l in out.splitlines() if l.startswith("{")][-1])
+        files = sorted(glob.glob(str(tmp_path / str(i) / "*.npy")))
+        dumps.append({os.path.basename(f): np.load(f) for f in files})
+        assert sum(os.path.getsize(f) for f in files) <= 64 * 10 ** 6
+        assert all(a.dtype in (np.float32, np.float64) for a in dumps[-1].values())
+        assert float(dumps[-1]["loss.npy"]) == np.float32(rec["loss"])
+        assert dumps[-1]["blocks.0.spectral.npy"].shape[-1] == 2 and "linear1.W.npy" in dumps[-1]
+    assert dumps[0].keys() == dumps[1].keys()
+    for k in dumps[0]:
+        assert np.array_equal(dumps[0][k], dumps[1][k]), k
+
+
+def test_bench_dump_outputs_samples_within_the_limit(tmp_path, monkeypatch):
+    import importlib.util
+    import torch
+    spec = importlib.util.spec_from_file_location("bench_main", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    monkeypatch.setattr(bench, "DUMP_LIMIT", 1 << 20)
+    arrays = {"big": torch.arange(1 << 20, dtype=torch.float32), "w": torch.randn(3, 4, dtype=torch.complex64),
+              "loss": torch.tensor(0.5, dtype=torch.float64)}
+    for i in range(2):
+        bench.dump_outputs(str(tmp_path / str(i)), arrays)
+    assert sum(os.path.getsize(f) for f in glob.glob(str(tmp_path / "0" / "*.npy"))) <= 1 << 20
+    big = np.load(tmp_path / "0" / "big.npy")
+    assert big.ndim == 1 and 0.9 * (1 << 18) < big.size < 1 << 18     # what the small arrays leave of 1 MiB
+    assert np.all(np.diff(big) > 0)                                   # distinct elements, in order
+    assert np.array_equal(big, np.load(tmp_path / "1" / "big.npy"))
+    w = np.load(tmp_path / "0" / "w.npy")
+    assert w.dtype == np.float32 and np.array_equal(w, torch.view_as_real(arrays["w"]).numpy())
+    loss = np.load(tmp_path / "0" / "loss.npy")
+    assert loss.dtype == np.float64 and float(loss) == 0.5

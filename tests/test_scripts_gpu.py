@@ -56,3 +56,22 @@ def test_two_phase_trainer_default_shape_runs_on_the_fused_engine(tmp_path):
     assert "resumed from epoch 2" in log
     log = _run(["training/two_phase/test_two_phase.py", "--sample", "5", "--out-dir", out], n)
     assert "Saved data sample!" in log
+
+
+def test_bench_dump_outputs_fused(tmp_path):
+    """bench.py --dump-outputs on the fused engine: the loss of the last timed step and the canonical parameters."""
+    import json
+    import numpy as np
+    out = tmp_path / "dump"
+    r = subprocess.run([sys.executable, "bench.py", "--gpus", "1", "--steps", "2", "--warmup", "3", "--grid", "32",
+                        "--modes", "4", "4", "4", "10", "--blocks", "2", "--no-e2e", "--dump-outputs", str(out)],
+                       cwd=ROOT, capture_output=True, text=True, timeout=600)
+    assert r.returncode == 0, r.stdout[-3000:] + "\n" + r.stderr[-3000:]
+    rec = json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][-1])
+    assert rec["impl"] == "fused" and rec["steps"] == 2
+    got = {p.name: np.load(p) for p in out.glob("*.npy")}
+    assert float(got["loss.npy"]) == np.float32(rec["loss"])
+    assert sum(p.stat().st_size for p in out.glob("*.npy")) <= 64 * 10 ** 6
+    for k in range(2):                  # [i, o, KX, KY, KZ, mt] complex -> trailing (real, imaginary)
+        assert got[f"blocks.{k}.spectral.npy"].shape == (20, 20, 8, 8, 8, 10, 2)
+    assert all(a.dtype == np.float32 and np.isfinite(a).all() for a in got.values())
